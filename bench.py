@@ -1,8 +1,13 @@
 #!/usr/bin/env python
 """bench.py — MIG placement decisions/s of the B200 placement engine on the BASELINE configurations.
 
-    python bench.py [--config c4] [--gpus N] [--steps K] [--warmup W] [--impl reference] [--min-age A]
+    python bench.py [--config c4] [--gpus N] [--steps K] [--warmup W] [--impl reference] [--min-age A] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR (configs c1-c4): after the timed steps, what the headline path computed in its last timed step, as float64 .npy
+files: result_gpu / result_start / result_size / result_status (one entry per request, in request order) and occupancy (the final
+occupancy byte of every GPU).  The workloads are seeded, so two builds of the project run with the same arguments can be compared
+output for output.  c5 is not supported: how its requests are grouped into calls depends on the host clock.
 
 --config (default c4, the configuration BASELINE.json's metric is quoted on; the others make every BASELINE config
 driver-reachable with the same parity / cpu_baseline / roofline / e2e keys):
@@ -211,6 +216,19 @@ class Ctx:
         return total_ms, wall
 
 
+def dump_outputs(out_dir, results, occupancy):
+    """--dump-outputs: every field of the result records and the final occupancy, as float64 (exact for every u8 / u16 / u32 value)."""
+    arrays = {"result_" + f: results[f] for f in results.dtype.names}
+    arrays["occupancy"] = occupancy
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    if total > 64 << 20:
+        raise SystemExit("--dump-outputs: %d bytes exceed the 64 MiB budget" % total)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
 def base_line(ctx, config, value, ms_per_step, config_extra, parity, launches, clocks, scaling="strong"):
     a = ctx.args
     cfg = {"workload": WORKLOADS[config], "l2": "flushed between timed steps (256 MiB write)", "timing": "cuda events per step on the launching stream, max over ranks",
@@ -376,6 +394,8 @@ def run_single_batch(ctx, config):
     line["roofline"] = roofline
     if cpu:
         line["cpu_baseline"] = cpu
+    if a.dump_outputs and ctx.rank == 0:
+        dump_outputs(a.dump_outputs, got_dev, occ_dev)
     eng.close()
     return line, parity
 
@@ -702,6 +722,8 @@ def run_c4(ctx):
         line["roofline"] = roofline
         line["cpu_baseline"] = cpu
         line.update(lines_extra)
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, np.concatenate(head["got"]), head["occ"])
         eng.close()
         return line, parity
 
@@ -791,6 +813,8 @@ def run_c4(ctx):
                             "phase_ms_per_step_max_over_ranks": {"pre-pass + pipeline (enqueue to kernel end)": ms_pipe, "occupancy all-gather (NCCL) + copy back": float(ph[1].item()),
                                                                   "result merge": 0.0}}
         line["cpu_baseline"] = cpu
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, np.concatenate(got_dev), occ_dev)
     dist.barrier()
     eng.close()
     return line, parity
@@ -909,7 +933,12 @@ def main():
     ap.add_argument("--min-age", type=int, default=1, help="c4: a FREE names an allocation at least this many batches old = batches in flight of the causal feed")
     ap.add_argument("--faithful-ops", type=int, default=10000, help="c4: operations of the churn prefix the reference-as-written port is timed on (SURVEY 8d)")
     ap.add_argument("--seconds", type=float, default=10.0, help="c5: length of the replay")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="c1-c4: write the results of the last timed step and the final occupancy to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "own" or args.config == "c5"):
+        ap.error("--dump-outputs needs --impl own and one of the configs c1-c4")
     args.warmup = max(args.warmup, 3) if args.impl == "own" else args.warmup
     sys.exit(run_reference(args) if args.impl == "reference" else run_own(args))
 
