@@ -1929,13 +1929,15 @@ __global__ void __launch_bounds__(kPipeThreads, 1) k_pipeline(CandTab tab, PipeA
                 {   // Two candidates for the next entry: the Newton step (hn) and plain chaining (the exit of the stage in front as it is).  Where a
                     // batch's contested front reaches far the Newton step over-corrects round after round; each stage uses the rule whose
                     // candidate of the PREVIOUS round came closer to what the stage in front has published now (study, section 8).
+                    // The candidates of round 1 are not scored: they come from the occupancy guess, and judging the rules by them sends
+                    // stages to plain chaining too early (batch 8 of config 4: 24 -> 19 rounds).
                     const uint32_t xp = tid < ISL_MAX_PROFILES ? s_specXp[tid] : 0u;
                     uint32_t ea = 0, eb = 0;
                     if (tid < ISL_MAX_PROFILES && s_havepred) { ea = (uint32_t)abs((int)s_predA[tid] - (int)xp); eb = (uint32_t)abs((int)s_predB[tid] - (int)xp); }
                     ea = __reduce_add_sync(0xFFFFFFFFu, ea); eb = __reduce_add_sync(0xFFFFFFFFu, eb);
                     __syncwarp();
                     if (tid < ISL_MAX_PROFILES) { s_predA[tid] = hn; s_predB[tid] = xp; }
-                    if (tid == 0) s_havepred = 1;
+                    if (tid == 0 && rnd >= 2) s_havepred = 1;
                     if (eb < ea) hn = xp;
                 }
                 if (tid < ISL_MAX_PROFILES) s_specH[tid] = hn;

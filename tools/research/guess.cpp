@@ -65,6 +65,17 @@ int main(int argc, char** argv) {
         auto cq = [&](const Heads& h) { long c = 0; for (int p : big) c += h[p]; return c; };
         auto cr = [&](const Heads& h) { long c = 0; for (int p : small) c += (long)h[p] * psize(p); return c; };
         std::vector<double> lq(S, 1.0), lr(S, 1.0); std::vector<long> peq(S), pxq(S), per(S), pxr(S); std::vector<bool> have(S, false);
+        // the pair of the small group (its longest single-slice and wider queue) and the hungry test of LEAD: the wider profile's pending request
+        // is more than LEAD request-times older than the single-slice one's at both ends of the segment
+        int pl = -1, ph = -1; for (int p : small) { if (psize(p) == 1 && (pl < 0 || q[p].size() > q[pl].size())) pl = p; if (psize(p) > 1 && (ph < 0 || q[p].size() > q[ph].size())) ph = p; }
+        const long lead_th = getenv("LEAD") ? atol(getenv("LEAD")) : -1;
+        auto lead = [&](const Heads& hh) { long t1 = hh[pl] < q[pl].size() ? (long)q[pl][hh[pl]] : (long)n, t2 = hh[ph] < q[ph].size() ? (long)q[ph][hh[ph]] : (long)n; return t1 - t2; };
+        // EXPERT variants: DMASS=1 the Newton candidate's mass target is the sum of the masses the stages in front consumed (what the device
+        // can compute from the D records) instead of this round's new entry of the stage in front; SCORE1=1 the candidates of round 1 are scored
+        // too (the device before r03); LEADLAG=1 the pass-through uses the change of the exit in front since the previous round (observable
+        // without a same-round prefix) instead of the change of its entry this round
+        const bool dmass = getenv("DMASS") != nullptr, score1 = getenv("SCORE1") != nullptr, leadlag = getenv("LEADLAG") != nullptr;
+        std::vector<Heads> Ep(S + 1, h0);
         const int secant = getenv("SECANT") ? atoi(getenv("SECANT")) : 0;
         std::vector<Heads> predA(S + 2), predB(S + 2); std::vector<bool> havePred(S + 2, false);
         std::vector<Heads> pH(S), pE(S); std::vector<bool> haveR(S, false); std::vector<double> lam(S, getenv("LAM0") ? atof(getenv("LAM0")) : 0.0);
@@ -100,17 +111,26 @@ int main(int argc, char** argv) {
             if (getenv("VERBM") && (int)b == atoi(getenv("VERBM"))) printf("      round %d: max %lu at stage %u (second %lu), mean busy %.0f, frontier %u\n", rounds, maxw, maxs, second, nb_ ? (double)sumw / nb_ : 0.0, frontier);
             crit += maxw;
             Hn[0] = h0;
+            auto hungry_at = [&](uint32_t s) { return lead_th >= 0 && pl >= 0 && ph >= 0 && lead(H[s]) > lead_th && lead(E[s + 1]) > lead_th; };
+            std::vector<long> sumDq(S + 1, 0), sumDr(S + 1, 0);
+            for (uint32_t s = 0; s < S; ++s) { sumDq[s + 1] = sumDq[s] + cq(E[s + 1]) - cq(H[s]); sumDr[s + 1] = sumDr[s] + cr(E[s + 1]) - cr(H[s]); }
             for (uint32_t s = 0; s < S; ++s) {
                 Hn[s + 1] = E[s + 1];
-                if (getenv("EXPERT") && rounds >= 2) {
+                if (getenv("EXPERT") && rounds >= (score1 ? 1 : 2)) {
                     // candidates for stage s+1's next entry
                     Heads A = E[s + 1];
                     { long dq = 0, dr = 0; for (int p : big) dq += (long)Hn[s][p] - (long)H[s][p]; for (int p : small) dr += ((long)Hn[s][p] - (long)H[s][p]) * psize(p);
+                      if (dmass) { dq = sumDq[s + 1] - cq(E[s + 1]); dr = sumDr[s + 1] - cr(E[s + 1]); }
                       long nb = 0, ns = 0; for (int p : big) nb += q[p].size(); for (int p : small) ns += (long)q[p].size() * psize(p);
                       auto clampadd = [&](int p, long d) { long v = (long)A[p] + d; v = std::max(0l, std::min<long>(v, q[p].size())); A[p] = v; };
                       { std::vector<int> b2 = big; long d = dq, tot = nb; std::sort(b2.begin(), b2.end()); for (size_t i = 0; i < b2.size(); ++i) { int p = b2[i]; long dp = i + 1 == b2.size() ? d : (tot ? std::lround((double)d * q[p].size() / tot) : 0); clampadd(p, dp); d -= dp; tot -= q[p].size(); } }
                       { std::vector<int> grp = small; long d = dr, tot = ns; std::sort(grp.begin(), grp.end(), [&](int x, int y) { return psize(x) > psize(y) || (psize(x) == psize(y) && x < y); });
                         for (size_t i = 0; i < grp.size(); ++i) { int p = grp[i]; long w = psize(p); long dp = i + 1 == grp.size() ? d / w : (tot ? std::lround((double)d * q[p].size() / tot) : 0); clampadd(p, dp); d -= dp * w; tot -= (long)q[p].size() * w; } } }
+                    if (s > 0 && hungry_at(s)) {
+                        // hungry stage in front: the split inside the small group passes through it, so its exit moves as its entry does
+                        for (int p : small) { long sh = leadlag ? (long)E[s + 1][p] - (long)Ep[s + 1][p] : (long)Hn[s][p] - (long)H[s][p];
+                            long v = (long)E[s + 1][p] + sh; A[p] = (uint32_t)std::max(0l, std::min<long>(v, q[p].size())); }
+                    }
                     Heads Bc = E[s + 1];
                     // which rule would have predicted this round's entry better last round?  errA[s+1], errB[s+1] were recorded then
                     auto dist = [&](const Heads& x, const Heads& y) { long d = 0; for (int p = 0; p < np; ++p) d += std::labs((long)x[p] - (long)y[p]); return d; };
@@ -150,13 +170,7 @@ int main(int argc, char** argv) {
                     if (getenv("LEAD")) {
                         // hungry regime: the heavier small profile's pending request is much older than the lighter one's at both ends of the segment ->
                         // it takes every span it can use, the split inside the group passes through the segment unchanged
-                        const long th = atol(getenv("LEAD"));
-                        int pl = -1, ph = -1; for (int p : small) { if (psize(p) == 1 && (pl < 0 || q[p].size() > q[pl].size())) pl = p; if (psize(p) > 1 && (ph < 0 || q[p].size() > q[ph].size())) ph = p; }
-                        if (pl >= 0 && ph >= 0) {
-                            auto lead = [&](const Heads& hh) { long t1 = hh[pl] < q[pl].size() ? (long)q[pl][hh[pl]] : (long)n, t2 = hh[ph] < q[ph].size() ? (long)q[ph][hh[ph]] : (long)n; return t1 - t2; };
-                            const bool hungry = lead(H[s]) > th && lead(E[s + 1]) > th;
-                            if (hungry) { for (int p : small) { long v = (long)base_exit[p] + (long)Hn[s][p] - (long)H[s][p]; h[p] = (uint32_t)std::max(0l, std::min<long>(v, q[p].size())); } }
-                        }
+                        if (hungry_at(s)) { for (int p : small) { long v = (long)base_exit[p] + (long)Hn[s][p] - (long)H[s][p]; h[p] = (uint32_t)std::max(0l, std::min<long>(v, q[p].size())); } }
                     }
                     if (getenv("RESID")) {
                         // what the mass step did: m = h - base_exit; the entry shift was sh = Hn[s] - H[s]; residual r = sh - m (zero mass per group); pass lambda_s * r on
@@ -193,6 +207,7 @@ int main(int argc, char** argv) {
                 while (dr > 0) { int bp = -1; uint32_t bt = 0xFFFFFFFFu; for (int p : small) if (h[p] < q[p].size() && psize(p) <= dr && q[p][h[p]] < bt) { bt = q[p][h[p]]; bp = p; } if (bp < 0) break; ++h[bp]; dr -= psize(bp); }
                 while (dr < 0) { int bp = -1; long bt = -1; for (int p : small) if (h[p] > 0 && psize(p) <= -dr && (long)q[p][h[p] - 1] > bt) { bt = q[p][h[p] - 1]; bp = p; } if (bp < 0) break; --h[bp]; dr += psize(bp); }
             }
+            Ep = E;
             bool any = false; uint32_t wrong = 0;
             for (uint32_t s = 0; s <= S; ++s) { if (Hn[s] != H[s]) any = true; if (Hn[s] != truth[s]) ++wrong; H[s] = Hn[s]; }
             if (getenv("VERB") && (int)b == atoi(getenv("VERB"))) { printf("      err:"); for (uint32_t s = 0; s < 48 && s <= S; ++s) { long d = 0; for (int p = 0; p < np; ++p) d += std::labs((long)H[s][p] - (long)truth[s][p]); printf(" %ld", d); } printf("\n"); }
